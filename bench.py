@@ -7,7 +7,8 @@ Reddit-shaped synthetic graph (BASELINE.json configs[1]); one process per GPU.
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 5 --warmup 1      # the reference op sequence on host cores
 
-A step = one 512-seed batch through the whole hot path.  Prints ONE JSON line (rank 0).
+A step = one 512-seed batch through the whole hot path.  Prints ONE JSON line (rank 0).  --dump-outputs DIR writes
+the embeddings the timed path returned for its last step as DIR/embeddings.npy (float32), for comparing builds.
 """
 import argparse
 import json
@@ -19,6 +20,7 @@ import time
 import numpy as np
 import torch
 
+sys.dont_write_bytecode = True       # the tree may be read-only: leave it as it is
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -174,7 +176,7 @@ def main():
     ap.add_argument("--depth", type=int, default=int(os.environ.get("GS_PIPE_DEPTH", "4")),
                     help="graph runners / compute streams alternating in the pipelined front end")
     ap.add_argument("--no-partitioned", action="store_true", help="skip the node-partitioned measurement at N > 1")
-    ap.add_argument("--repeats", type=int, default=0,
+    ap.add_argument("--repeats", type=int, default=1,
                     help="how many times each K-step timed region is repeated (median reported); 0 = auto (~0.3 s per leg)")
     ap.add_argument("--no-config3", action="store_true", help="skip the short max-pool/bf16 pass behind roofline_tensor")
     ap.add_argument("--workload", default="reddit", choices=["reddit", "unsup", "rmat", "train"],
@@ -182,7 +184,11 @@ def main():
                          "step, node-partitioned, data parallel; rmat = configs[4]: R-MAT graph, CSR sampler, partitioned")
     ap.add_argument("--rmat-scale", type=int, default=20, help="log2 of the R-MAT id space (27 = BASELINE configs[4])")
     ap.add_argument("--rmat-nodes", type=int, default=0, help="nodes after trimming (0 = 2^scale; 100000000 for configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's output embeddings to DIR/embeddings.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "reddit"):
+        ap.error("--dump-outputs covers the CUDA path of the reddit workload")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -296,12 +302,12 @@ def main():
         #      own streams (steps are independent), so one step's sampler + gather overlaps the previous step's GEMMs
         pipe = mdl.pipelined(BATCH, normalize=True, depth=args.depth)
         cur = torch.cuda.current_stream(dev)
+        clocks = ClockSampler(local_rank)      # NVML start-up perturbs the steps around it: keep it in the warm-up
+        clocks.start()
         for i in range(args.warmup):
             pipe.submit_device(seeds_dev[i])
         pipe.synchronize()
         barrier()
-        clocks = ClockSampler(local_rank)
-        clocks.start()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ms_value = []
         for rep in range(reps):
@@ -312,13 +318,14 @@ def main():
             for c in pipe.computes:
                 c.wait_event(e0)
             for i in range(args.steps):
-                pipe.submit_device(seeds_dev[base + i])
+                out = pipe.submit_device(seeds_dev[base + i])
             for c in pipe.computes:
                 cur.wait_stream(c)
             e1.record(cur)
             pipe.synchronize()
             barrier()
             ms_value.append(max_over_ranks(e0.elapsed_time(e1)))
+        last_output = out.float().cpu().numpy() if args.dump_outputs else None   # the last timed step's result
         clk = clocks.summary()
         launches_per_step = pipe.runners[0].launches_per_replay
         pipe.close()
@@ -340,7 +347,7 @@ def main():
         kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in pev]))
         res = dict(ms_value=stats(ms_value), clocks=clk, launches=launches_per_step * args.steps,
                    launches_per_step=launches_per_step, ms_probe_step=ms_probe_total / n_probe,
-                   gather_kernel_ms=max_over_ranks(kernel_ms), reps=reps)
+                   gather_kernel_ms=max_over_ranks(kernel_ms), reps=reps, last_output=last_output)
         res["ms_total"] = res["ms_value"]["median"]
         res["value"] = world * BATCH * args.steps / (res["ms_total"] * 1e-3)
         if not do_e2e:
@@ -478,6 +485,7 @@ def main():
                 out["nvlink_note"] = "unique remote rows of one step x row bytes / pipelined step time (lower bound on the fetch pass's rate)"
             if full:
                 out.update({"e2e": pr["e2e"], "e2e_ms_per_step": pr["ms_e2e"] / args.steps, "value_spread_ms": pr["ms_value"],
+                            "last_output": pr["last_output"],
                             "clocks": pr["clocks"], "launches": pr["launches"],
                             "partition": "community-aligned contiguous ranges, %d..%d rows per GPU" % (
                                 min(np.diff(bounds)), max(np.diff(bounds))),
@@ -507,6 +515,10 @@ def main():
     if rank != 0:
         return
     head = part if part is not None else None
+    last_output = (head if head is not None else rep).pop("last_output")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "embeddings.npy"), last_output)
     roof = (tensor_roofline(rep) if kind == "maxpool" else hbm_roofline(rep)) if rep["gather_kernel_ms"] > 0 else None
     cpu = None
     if world == 1 and args.cpu_batches > 0:

@@ -1,12 +1,12 @@
 """Generate tests/golden/*.npz by executing the reference's own hot-path python
-(/root/reference/graphsage/{neigh_samplers,aggregators,layers,inits,models,minibatch}.py)
-under the numpy TF shim (tf_shim.py).  Run HERE (the container that has
-/root/reference); the GPU box only reads the committed .npz files.
+(graphsage/{neigh_samplers,aggregators,layers,inits,models,minibatch}.py of a williamleif/GraphSAGE
+checkout) under the numpy TF shim (tf_shim.py).  The tests only read the committed .npz files.
 
-    python tests/golden/make_golden.py
+    GRAPHSAGE_REFERENCE=<checkout of williamleif/GraphSAGE> python tests/golden/make_golden.py [name]
 
-Nothing from /root/reference is copied: the modules are imported from where they lie.
+Nothing from the reference is copied: the modules are imported from where they lie.
 """
+import json
 import os
 import sys
 import types
@@ -15,9 +15,12 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
+REFERENCE = os.environ.get("GRAPHSAGE_REFERENCE", "")
+if not os.path.isdir(os.path.join(REFERENCE, "graphsage")):
+    sys.exit("set GRAPHSAGE_REFERENCE to a checkout of williamleif/GraphSAGE")
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, REFERENCE)
 
 import tf_shim  # noqa: E402
 
@@ -351,6 +354,60 @@ def golden_heads():
     save("heads", **out)
 
 
+def golden_toy_ppi(quota=(1500, 300, 500)):
+    """A sample of the reference's example_data/toy-ppi small enough to commit: for train, val and test nodes in turn, a
+    breadth-first ball (neighbours in id order) from the first node of that kind, grown until it holds `quota` nodes,
+    then the induced subgraph.  Node ids, flags, links (in file order, with their flags), features and labels keep the
+    file's values; tests/test_data_cpu.py writes them back out in the file format."""
+    prefix = os.path.join(REFERENCE, "example_data", "toy-ppi")
+    with open(prefix + "-G.json") as fp:
+        g = json.load(fp)
+    nodes, links = g["nodes"], g["links"]
+    kind = np.array([2 if nd["test"] else 1 if nd["val"] else 0 for nd in nodes])
+    nbrs = [[] for _ in nodes]
+    for ln in links:
+        nbrs[ln["source"]].append(ln["target"])
+        nbrs[ln["target"]].append(ln["source"])
+    keep = set()
+    for k, q in enumerate(quota):
+        taken = []
+        for start in np.nonzero(kind == k)[0]:
+            if len(taken) == q:
+                break
+            if int(start) in keep:
+                continue
+            frontier = [int(start)]
+            keep.add(int(start))
+            taken.append(int(start))
+            while frontier and len(taken) < q:
+                nxt = []
+                for u in frontier:
+                    for v in sorted(set(nbrs[u])):
+                        if v not in keep and len(taken) < q:
+                            keep.add(v)
+                            taken.append(v)
+                            nxt.append(v)
+                frontier = nxt
+    pos = sorted(keep)
+    row = {p: i for i, p in enumerate(pos)}
+    sub = [ln for ln in links if ln["source"] in row and ln["target"] in row]
+    feats = np.load(prefix + "-feats.npy")[pos]
+    with open(prefix + "-id_map.json") as fp:
+        id_map = json.load(fp)
+    with open(prefix + "-class_map.json") as fp:
+        class_map = json.load(fp)
+    ids = [nodes[p]["id"] for p in pos]
+    assert all(id_map[str(i)] == p for i, p in zip(ids, pos))
+    assert set(np.unique(feats)) <= {0.0, 1.0}
+    save("toy_ppi", ids=np.array(ids, np.int32), val=np.array([nodes[p]["val"] for p in pos]),
+         test=np.array([nodes[p]["test"] for p in pos]),
+         feats=feats.astype(np.uint8), labels=np.array([class_map[str(i)] for i in ids], np.uint8),
+         link_source=np.array([row[ln["source"]] for ln in sub], np.int16),
+         link_target=np.array([row[ln["target"]] for ln in sub], np.int16),
+         link_train_removed=np.array([ln["train_removed"] for ln in sub]),
+         link_test_removed=np.array([ln["test_removed"] for ln in sub]), graph_name=g["graph"]["name"])
+
+
 def _standalone(fn):
     """meanpool / iterators / heads were added after the first four fixtures: each starts from a fresh initialiser
     stream, so regenerating everything reproduces every committed file."""
@@ -359,7 +416,7 @@ def _standalone(fn):
 
 
 if __name__ == "__main__":
-    later = {"meanpool": golden_meanpool, "iterators": golden_iterators, "heads": golden_heads}
+    later = {"meanpool": golden_meanpool, "iterators": golden_iterators, "heads": golden_heads, "toy_ppi": golden_toy_ppi}
     if len(sys.argv) > 1:
         _standalone(later[sys.argv[1]])
         sys.exit(0)

@@ -5,6 +5,7 @@ The iterator fixtures in tests/golden/iterators.npz were produced by the referen
 (tests/golden/make_golden.py: golden_iterators) running over graphsage_b200.graph.Graph with numpy's legacy global
 generator seeded as noted there; these tests replay the same seeds through graphsage_b200.minibatch.
 """
+import json
 import os
 import random
 
@@ -17,7 +18,7 @@ from graphsage_b200 import minibatch, utils  # noqa: E402
 from graphsage_b200.graph import Graph, node_link_graph, to_csr  # noqa: E402
 
 GOLD = os.path.join(HERE, "golden", "iterators.npz")
-TOY = "/root/reference/example_data/toy-ppi"
+TOY_GOLD = os.path.join(HERE, "golden", "toy_ppi.npz")
 
 
 def fixture_graph():
@@ -258,13 +259,34 @@ def test_random_walk_pairs():
     assert all(H.degree(a) > 0 for a in per_start)
 
 
-@pytest.mark.skipif(not os.path.exists(TOY + "-G.json"), reason="reference example_data not present on this machine")
-def test_toy_ppi_ingest_and_tables():
-    G, feats, id_map, walks, class_map = utils.load_data(TOY, normalize=True, load_walks=False)
-    assert len(G) == 14755 and len(G.edges()) == 228431 and feats.shape == (14755, 50) and len(id_map) == 14755
+@pytest.fixture(scope="module")
+def toy(tmp_path_factory):
+    """tests/golden/toy_ppi.npz - a 2,300-node sample of the reference's example_data/toy-ppi (make_golden.py:
+    golden_toy_ppi) - written back out in that dataset's file format; returns the path prefix."""
+    t = np.load(TOY_GOLD)
+    ids, feats, labels = [int(i) for i in t["ids"]], t["feats"].astype(np.float64), t["labels"].tolist()
+    nodes = [{"test": bool(te), "id": i, "feature": f.tolist(), "val": bool(va), "label": lab}
+             for i, va, te, f, lab in zip(ids, t["val"], t["test"], feats, labels)]
+    links = [{"test_removed": bool(te), "train_removed": bool(tr), "target": int(d), "source": int(s)}
+             for s, d, tr, te in zip(t["link_source"], t["link_target"], t["link_train_removed"], t["link_test_removed"])]
+    prefix = str(tmp_path_factory.mktemp("toy") / "toy-ppi")
+    with open(prefix + "-G.json", "w") as fp:
+        json.dump({"directed": False, "graph": {"name": str(t["graph_name"])}, "nodes": nodes, "links": links,
+                   "multigraph": False}, fp)
+    with open(prefix + "-id_map.json", "w") as fp:
+        json.dump({str(i): r for r, i in enumerate(ids)}, fp)
+    with open(prefix + "-class_map.json", "w") as fp:
+        json.dump({str(i): lab for i, lab in zip(ids, labels)}, fp)
+    np.save(prefix + "-feats.npy", feats)
+    return prefix
+
+
+def test_toy_ppi_ingest_and_tables(toy):
+    G, feats, id_map, walks, class_map = utils.load_data(toy, normalize=True, load_walks=False)
+    assert len(G) == 2300 and len(G.edges()) == 41857 and feats.shape == (2300, 50) and len(id_map) == 2300
     assert len(next(iter(class_map.values()))) == 121 and isinstance(next(iter(id_map)), int)
     kinds = [(G.node[n]["val"], G.node[n]["test"]) for n in G.nodes()]
-    assert kinds.count((False, False)) == 9716 and kinds.count((True, False)) == 1825 and kinds.count((False, True)) == 3214
+    assert kinds.count((False, False)) == 1500 and kinds.count((True, False)) == 300 and kinds.count((False, True)) == 500
     tr = np.array([id_map[n] for n in G.nodes() if not G.node[n]["val"] and not G.node[n]["test"]])
     assert np.allclose(feats[tr].mean(axis=0), 0, atol=1e-9)
     np.random.seed(123)
@@ -286,14 +308,14 @@ def test_toy_ppi_ingest_and_tables():
     assert all(it.deg[id_map[u]] > 0 for u in it.train_nodes)
 
 
-@pytest.mark.skipif(not os.path.exists(TOY + "-G.json"), reason="reference example_data not present on this machine")
-def test_config1_toy_ppi_cpu_oracle_path_loss_decreases():
+def test_config1_toy_ppi_cpu_oracle_path_loss_decreases(toy):
     """SURVEY 8d config 1: toy-ppi, graphsage_mean, B = 512, max_degree 128, dims [50, 128, 128], 121 sigmoid classes,
     fanouts [25, 10], lr 0.01 (reference supervised_train.py:32-49) on the CPU oracle path (oracle/torch_ref.py):
-    ingest -> iterator -> sample -> gather -> aggregate -> l2-normalise -> Dense head -> sigmoid xent -> clipped Adam."""
+    ingest -> iterator -> sample -> gather -> aggregate -> l2-normalise -> Dense head -> sigmoid xent -> clipped Adam.
+    The sample's train nodes last three batches, so the steps run over epochs, reshuffled as supervised_train.py does."""
     import torch
     from oracle import torch_ref
-    G, feats, id_map, _, class_map = utils.load_data(TOY, normalize=True)
+    G, feats, id_map, _, class_map = utils.load_data(toy, normalize=True)
     np.random.seed(123)
     it = minibatch.NodeMinibatchIterator(G, id_map, None, class_map, 121, batch_size=512, max_degree=128)
     n, F, D, C = len(id_map), feats.shape[1], 128, 121
@@ -313,6 +335,8 @@ def test_config1_toy_ppi_cpu_oracle_path_loss_decreases():
     it.shuffle()
     losses = []
     for step in range(12):
+        if it.end():
+            it.shuffle()
         feed, labels = it.next_minibatch_feed_dict()
         seeds = torch.tensor(feed["batch"], dtype=torch.int32)
         out = torch_ref.forward(adj_t, feats_t, seeds, [25, 10], aggs, True, "mean", 123, 2 * step, normalize=True)
