@@ -6,7 +6,7 @@ All compute goes through libgraphsage_b200.so (include/graphsage_b200.h); there 
 """
 from . import _lib, aggregators, graph, inits, layers, minibatch, models, neigh_samplers, ops, prediction, utils  # noqa: F401
 from .aggregators import (GCNAggregator, MaxPoolingAggregator, MeanAggregator, MeanPoolingAggregator,  # noqa: F401
-                          set_default_math)
+                          SeqAggregator, set_default_math)
 from .layers import Dense, Layer, identity, relu  # noqa: F401
 from .models import SAGEInfo, SampleAndAggregate  # noqa: F401
 from .neigh_samplers import CSRNeighborSampler, UniformNeighborSampler  # noqa: F401

@@ -93,6 +93,8 @@ _SIGNATURES = {
                                       c_vp]),
     "gs_pipeline_step": (c_i32, [c_vp, c_vp, c_i64, ctypes.POINTER(c_vp), c_i32, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp,
                                  c_vp, c_vp]),
+    "gs_row_used": (c_i32, [c_vp, c_i32, c_i64, c_i32, c_i64, c_vp, c_vp]),
+    "gs_lstm_seq": (c_i32, [c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "gs_l2_normalize_rows": (c_i32, [c_vp, c_i64, c_i32, c_i64, c_vp]),
     "gs_bump_counter": (c_i32, [c_vp, c_u64, c_vp]),
 }

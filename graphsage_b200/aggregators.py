@@ -1,5 +1,5 @@
-"""MeanAggregator / GCNAggregator / MaxPoolingAggregator - the surface of reference
-graphsage/aggregators.py:6-195 over the B200 kernels.
+"""MeanAggregator / GCNAggregator / MaxPoolingAggregator / MeanPoolingAggregator / SeqAggregator - the surface of
+reference graphsage/aggregators.py over the B200 kernels.
 
 Two entry points per aggregator:
   agg((self_vecs[n, in], neigh_vecs[n, k, neigh_in])) -> [n, out * (2 if concat else 1)]
@@ -308,6 +308,122 @@ class MaxPoolingAggregator(_SageAggregator):
                 xs[s.out_row0:s.out_row0 + n] = src[s.self_row0:s.self_row0 + n]
         return self._finish([(xs, self.input_dim, self.vars["self_weights"]),
                              (hmax, self.hidden_dim, self.vars["neigh_weights"])], self._combine())
+
+
+class SeqAggregator(_SageAggregator):
+    """act(concat_or_add(self @ Ws, h_{len-1} @ Wn)) with h the outputs of an LSTM run over the neighbour rows in sampled
+    order - reference graphsage/aggregators.py:363-449.  BasicLSTMCell(H), H = 128 ("small") / 256 ("big"); len = the
+    number of non-zero neighbour rows (at least 1), and the LSTM consumes the FIRST len rows (dynamic_rnn's
+    sequence_length), zero rows included.
+
+    The cell's kernel [neigh_in + H, 4H] (gate columns i, j, f, o) and bias [4H] live in `cell_vars`, not in `vars`: the
+    reference keeps them in the cell, so they are trained but not weight-decayed.  Like the reference, the aggregator
+    stores `dropout` but never applies it.  Kernels per hop: gather of the neighbour rows (layer 0), the input projection
+    on gs_sage_gemm, gs_lstm_seq for the recurrence, then gs_sage_gemm for the two matmuls, combine, bias and act."""
+
+    def __init__(self, input_dim, output_dim, model_size="small", neigh_input_dim=None, dropout=0., bias=False,
+                 act=relu, name=None, concat=False, device="cuda", **kwargs):
+        super(SeqAggregator, self).__init__(**kwargs)
+        self.dropout = dropout
+        self.bias = bias
+        self.act = act
+        self.concat = concat
+        if neigh_input_dim is None:
+            neigh_input_dim = input_dim
+        if model_size == "small":
+            hidden_dim = self.hidden_dim = 128
+        elif model_size == "big":
+            hidden_dim = self.hidden_dim = 256
+        else:
+            raise ValueError("model_size must be 'small' or 'big'")
+        self.vars["neigh_weights"] = glorot([hidden_dim, output_dim], name="neigh_weights", device=device)
+        self.vars["self_weights"] = glorot([input_dim, output_dim], name="self_weights", device=device)
+        if self.bias:   # the reference reads self.output_dim before setting it here (aggregators.py:394-395); fixed
+            self.vars["bias"] = zeros([output_dim * (2 if concat else 1)], name="bias", device=device)
+        # BasicLSTMCell variables: TF's get_variable default (glorot uniform over the full shape), zero bias
+        self.cell_vars = {"kernel": glorot([neigh_input_dim + hidden_dim, 4 * hidden_dim], name="kernel", device=device),
+                          "bias": zeros([4 * hidden_dim], name="bias", device=device)}
+        self.input_dim = input_dim
+        self.output_dim = output_dim
+        self.neigh_input_dim = neigh_input_dim
+        self.math = _DEFAULT_MATH[0]
+
+    def parameters(self):
+        return list(self.vars.values()) + list(self.cell_vars.values())
+
+    def _combine(self):
+        return ops.COMBINE_CONCAT if self.concat else ops.COMBINE_ADD
+
+    def _cell_weights(self):
+        kernel = self.cell_vars["kernel"]
+        return kernel[:self.neigh_input_dim], kernel[self.neigh_input_dim:]
+
+    def _project(self, x):
+        """P = x @ kernel[:neigh_in] + cell bias: the input half of every gate pre-activation, for all steps at once."""
+        if getattr(self, "_packed_cell", None) is None:
+            self._packed_cell = ops.PackedWeights()
+        Wx, _ = self._cell_weights()
+        return ops.sage_gemm([(x, self.neigh_input_dim, Wx)], bias=self.cell_vars["bias"], act=ops.ACT_NONE,
+                             math=self.math, packed=self._packed_cell)
+
+    def _call(self, inputs):
+        self_vecs, neigh_vecs = inputs                      # dropout is stored but not applied (aggregators.py:405-449)
+        n, k, d = neigh_vecs.shape
+        x = neigh_vecs.reshape(n * k, d)
+        if x.stride(1) != 1:
+            x = x.contiguous()
+        used = ops.row_used(x)
+        neigh_h = ops.lstm_seq(self._project(x), self._cell_weights()[1], used, n, k)
+        return self._finish([(self_vecs, self.input_dim, self.vars["self_weights"]),
+                             (neigh_h, self.hidden_dim, self.vars["neigh_weights"])], self._combine())
+
+    def _used_table(self, src, persistent):
+        """used[] over the source rows.  The feature table (layer 0) is scanned once per tensor version, as
+        MaxPoolingAggregator._bf16_table casts it; intermediate activations are fresh buffers, scanned on every call."""
+        if not persistent:
+            return ops.row_used(src)
+        key = (src.data_ptr(), src._version, tuple(src.shape))
+        if getattr(self, "_used_ref", None) is not src or getattr(self, "_used_key", None) != key:
+            self._used, self._used_ref, self._used_key = ops.row_used(src), src, key
+        return self._used
+
+    def neighbour_rows(self, src, s):
+        """The n*k neighbour rows of segment s as an fp32 matrix (a view of src for range-addressed rows)."""
+        n, k = s.n, s.k
+        if s.neigh_ids is None and src.dtype == torch.float32:
+            return src[s.neigh_row0:s.neigh_row0 + n * k]
+        F = src.shape[1]
+        x = torch.empty((n * k, ops.pad_cols(F)), dtype=torch.float32, device=src.device)[:, :F]
+        if src.dtype == torch.float32:
+            return ops.gather_rows(src, s.neigh_ids[:n * k], out=x)
+        return ops.gather_rows_f32(src, ids=None if s.neigh_ids is None else s.neigh_ids[:n * k], row0=s.neigh_row0,
+                                   n=n * k, out=x)
+
+    def self_rows(self, src, segments, rows):
+        s0 = segments[0]
+        if len(segments) == 1 and s0.self_ids is None and s0.out_row0 == 0 and src.dtype == torch.float32:
+            return src[s0.self_row0:s0.self_row0 + s0.n]         # the self rows are already a dense fp32 row range
+        F = src.shape[1]
+        xs = torch.empty((rows, ops.pad_cols(F)), dtype=torch.float32, device=src.device)[:, :F]
+        for s in segments:
+            ops.gather_rows_f32(src, ids=None if s.self_ids is None else s.self_ids[:s.n], row0=s.self_row0, n=s.n,
+                                out=xs[s.out_row0:s.out_row0 + s.n])
+        return xs
+
+    def aggregate_rows(self, src, segments, final=None, src_persistent=False):
+        if hasattr(src, "c_table"):
+            raise NotImplementedError("the seq aggregator does not read node-partitioned (sharded) feature tables")
+        rows = max(s.out_row0 + s.n for s in segments)
+        used = self._used_table(src, src_persistent)
+        Wh = self._cell_weights()[1]
+        neigh_h = torch.empty((rows, self.hidden_dim), dtype=torch.float32, device=src.device)
+        for s in segments:
+            P = self._project(self.neighbour_rows(src, s))
+            ops.lstm_seq(P, Wh, used, s.n, s.k, row_ids=None if s.neigh_ids is None else s.neigh_ids[:s.n * s.k],
+                         row0=s.neigh_row0,
+                         out=neigh_h[s.out_row0:s.out_row0 + s.n])
+        return self._finish([(self.self_rows(src, segments, rows), self.input_dim, self.vars["self_weights"]),
+                             (neigh_h, self.hidden_dim, self.vars["neigh_weights"])], self._combine())
 
 
 class MeanPoolingAggregator(MaxPoolingAggregator):

@@ -9,7 +9,7 @@ from collections import namedtuple
 import torch
 
 from . import ops
-from .aggregators import GCNAggregator, MaxPoolingAggregator, MeanAggregator, MeanPoolingAggregator
+from .aggregators import GCNAggregator, MaxPoolingAggregator, MeanAggregator, MeanPoolingAggregator, SeqAggregator
 from .layers import identity, relu  # noqa: F401
 
 # reference graphsage/models.py:180-185
@@ -20,7 +20,7 @@ SAGEInfo = namedtuple("SAGEInfo",
                        "output_dim"])     # the output (i.e., hidden) dimension
 
 _AGGREGATORS = {"mean": MeanAggregator, "maxpool": MaxPoolingAggregator, "gcn": GCNAggregator,
-                "meanpool": MeanPoolingAggregator}
+                "meanpool": MeanPoolingAggregator, "seq": SeqAggregator}
 
 
 class SampleAndAggregate(object):
@@ -37,9 +37,6 @@ class SampleAndAggregate(object):
         for kwarg in kwargs.keys():
             assert kwarg in allowed_kwargs, "Invalid keyword argument: " + kwarg   # reference models.py:22-24
         if aggregator_type not in _AGGREGATORS:
-            if aggregator_type in ("seq",):
-                raise NotImplementedError("aggregator_type %r is outside the hot path (SURVEY section 2, row 5)"
-                                          % aggregator_type)
             raise ValueError("Unknown aggregator: %r" % (aggregator_type,))
         self.aggregator_cls = _AGGREGATORS[aggregator_type]
         if identity_dim > 0:
@@ -52,6 +49,8 @@ class SampleAndAggregate(object):
         self.model_size = model_size
         self.adj_info = adj
         if hasattr(features, "c_table"):                 # parallel.ShardedFeatures: node-partitioned table
+            if aggregator_type == "seq":
+                raise NotImplementedError("the seq aggregator does not read node-partitioned (sharded) feature tables")
             self.features = features
             self._finish_init(placeholders, adj, degrees, layer_infos, concat, model_size, identity_dim, device)
             return
@@ -127,7 +126,7 @@ class SampleAndAggregate(object):
                 act = identity if layer == L - 1 else relu                      # models.py:307-310
                 kw = dict(act=act, dropout=self.placeholders.get("dropout", 0.), name=name, concat=concat,
                           device=self.device)
-                if issubclass(self.aggregator_cls, MaxPoolingAggregator):
+                if issubclass(self.aggregator_cls, (MaxPoolingAggregator, SeqAggregator)):
                     kw["model_size"] = model_size
                 aggregators.append(self.aggregator_cls(dim_mult * dims[layer], dims[layer + 1], **kw))
         if any(getattr(a, "dropout", 0.) for a in aggregators):

@@ -541,6 +541,62 @@ def maxpool_mlp_fused(table, n_groups, k, W, bias, packed, row_ids=None, row0=0,
     return out
 
 
+def row_used(x, out=None):
+    """tf.sign(tf.reduce_max(tf.abs(x), axis=-1)) per row (reference graphsage/aggregators.py:411) as uint8 [rows]:
+    1 where the row has any non-zero element.  x: float32 or bfloat16, row-major [rows, F] (any row stride)."""
+    require_cuda(x, out)
+    if x.dim() != 2 or x.stride(1) != 1:
+        raise ValueError("x must be a row-major 2-D tensor")
+    n, F = x.shape
+    if out is None:
+        out = torch.empty((n,), dtype=torch.uint8, device=x.device)
+    if out.dtype != torch.uint8 or out.numel() < n or not out.is_contiguous():
+        raise ValueError("out must be a contiguous uint8 tensor with >= rows elements")
+    ev = _probe("row_used/%d" % n)
+    check(lib().gs_row_used(ptr(x), _dtype_code(x), n, F, x.stride(0), ptr(out), stream_ptr()))
+    _launched(1 if n else 0, ev)
+    return out
+
+
+def lstm_seq(P, Wh, used, n, k, row_ids=None, row0=0, out=None, keep=False):
+    """dynamic_rnn(BasicLSTMCell(H), sequence_length = max(1, sum(used))) and the gather of h_{len-1} (reference
+    graphsage/aggregators.py:408-433) for n sequences of k steps, in one launch of gs_lstm_seq.
+    P: float32 [n*k, >=4H] input projection (x @ kernel[:in] + bias); Wh: float32 [H, 4H] (kernel[in:]); used: uint8 rows
+    addressed by row_ids[g*k + t] (or row0 + g*k + t).  Returns out [n, H], or (out, keep_h, keep_c, lengths) with keep
+    (keep_h / keep_c [n, k, H] hold h_t / c_t for t < len; later steps are not written)."""
+    require_cuda(P, Wh, used, row_ids, out)
+    if P.dtype != torch.float32 or P.stride(1) != 1 or Wh.dtype != torch.float32:
+        raise TypeError("P and Wh must be row-major float32")
+    if used.dtype != torch.uint8:
+        raise TypeError("used must be uint8")
+    H = Wh.shape[0]
+    if Wh.shape[1] != 4 * H:
+        raise ValueError("Wh must be [H, 4H]")
+    Wh = Wh.contiguous()
+    n, k = int(n), int(k)
+    if P.shape[0] < n * k or P.shape[1] < 4 * H:
+        raise ValueError("P must be [>= n*k, >= 4H]")
+    if row_ids is not None:
+        row_ids = _i32(row_ids.reshape(-1), "row_ids")
+        if row_ids.numel() < n * k:
+            raise ValueError("row_ids shorter than n*k")
+    dev = P.device
+    if out is None:
+        out = torch.empty((n, H), dtype=torch.float32, device=dev)
+    if out.dtype != torch.float32 or out.stride(1) != 1 or out.shape[0] < n or out.shape[1] < H:
+        raise ValueError("out must be a row-major float32 [>= n, >= H] matrix")
+    keep_h = keep_c = lengths = None
+    if keep:
+        keep_h = torch.empty((n, k, H), dtype=torch.float32, device=dev)
+        keep_c = torch.empty((n, k, H), dtype=torch.float32, device=dev)
+        lengths = torch.empty((n,), dtype=torch.int32, device=dev)
+    ev = _probe("lstm_seq/%d" % n)
+    check(lib().gs_lstm_seq(ptr(P), P.stride(0), ptr(Wh), H, ptr(used), ptr(row_ids), int(row0), n, k, ptr(out),
+                            out.stride(0), ptr(keep_h), ptr(keep_c), ptr(lengths), stream_ptr()))
+    _launched(1 if n else 0, ev)
+    return (out, keep_h, keep_c, lengths) if keep else out
+
+
 def l2_normalize_rows_(x):
     """In-place tf.nn.l2_normalize(x, 1) - reference graphsage/models.py:368."""
     require_cuda(x)

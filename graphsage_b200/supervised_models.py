@@ -11,6 +11,7 @@ supervised_models.py:85-126.
 import torch
 
 from . import ops
+from .aggregators import MaxPoolingAggregator, SeqAggregator
 from .layers import act_code, identity, relu  # noqa: F401
 from .models import SampleAndAggregate
 
@@ -168,6 +169,104 @@ class _PoolAggregateRowsFn(torch.autograd.Function):
         return None, dsrc, None, dWs, dWn, dWm, dbm
 
 
+def lstm_seq_backward(P, X, Wx, Wh, keep_h, keep_c, lengths, dout, need_dx):
+    """BPTT through out = h_{len-1} of BasicLSTMCell over one hop's n sequences of k steps (reference
+    aggregators.py:408-433 backwards).  P [n*k, 4H] is the input projection, X [n*k, in] its input, keep_h / keep_c
+    [n, k, H] the states the forward kept (steps t >= len unspecified) and dout [n, H] the gradient of the outputs.
+    Gate activations are recomputed from P + h_{t-1} @ Wh; steps t >= len carry no gradient, and len none at all.
+    Returns (dWx, dWh, db, dX or None)."""
+    n, k, H = keep_h.shape
+    live = (torch.arange(k, device=P.device).unsqueeze(0) < lengths.long().unsqueeze(1)).unsqueeze(2)   # [n, k, 1]
+    hs = torch.where(live, keep_h, torch.zeros((), dtype=keep_h.dtype, device=keep_h.device))
+    cs = torch.where(live, keep_c, torch.zeros((), dtype=keep_c.dtype, device=keep_c.device))
+    h_prev = torch.cat([torch.zeros_like(hs[:, :1]), hs[:, :-1]], dim=1)
+    c_prev = torch.cat([torch.zeros_like(cs[:, :1]), cs[:, :-1]], dim=1)
+    G = P[:, :4 * H].reshape(n, k, 4 * H) + (h_prev.reshape(n * k, H) @ Wh).reshape(n, k, 4 * H)
+    gi, gj, gf, go = G.split(H, dim=2)
+    si, tj, sf, so = torch.sigmoid(gi), torch.tanh(gj), torch.sigmoid(gf + 1.0), torch.sigmoid(go)
+    tc = torch.tanh(cs)
+    last = lengths.long() - 1
+    dG = torch.zeros_like(G)
+    dh = torch.zeros((n, H), dtype=dout.dtype, device=dout.device)
+    dc = torch.zeros_like(dh)
+    for t in range(k - 1, -1, -1):
+        dh = dh + torch.where((last == t).unsqueeze(1), dout, torch.zeros((), dtype=dout.dtype, device=dout.device))
+        m = live[:, t].to(dout.dtype)
+        dh = dh * m
+        dc = (dc + dh * so[:, t] * (1.0 - tc[:, t] * tc[:, t])) * m
+        d_o = dh * tc[:, t] * so[:, t] * (1.0 - so[:, t])
+        d_i = dc * tj[:, t] * si[:, t] * (1.0 - si[:, t])
+        d_j = dc * si[:, t] * (1.0 - tj[:, t] * tj[:, t])
+        d_f = dc * c_prev[:, t] * sf[:, t] * (1.0 - sf[:, t])
+        dG[:, t] = torch.cat([d_i, d_j, d_f, d_o], dim=1)
+        dh = dG[:, t] @ Wh.t()
+        dc = dc * sf[:, t]
+    dP = dG.reshape(n * k, 4 * H)
+    dWh = h_prev.reshape(n * k, H).t() @ dP
+    return X.t() @ dP, dWh, dP.sum(dim=0), (dP @ Wx.t() if need_dx else None)
+
+
+class _SeqAggregateRowsFn(torch.autograd.Function):
+    """y = agg.aggregate_rows(src, segments) for SeqAggregator, differentiable w.r.t. self / neigh weights, the cell's
+    kernel and bias, and (layers >= 1) src.  The forward runs the inference kernels (gather, projection GEMM,
+    gs_lstm_seq, final GEMM) and keeps X, P, h_t, c_t and the lengths of every hop for the BPTT backward."""
+
+    @staticmethod
+    def forward(ctx, agg, src, segments, Ws, Wn, kernel, cbias):
+        code, post = act_code(agg.act)
+        if post is not None:
+            raise NotImplementedError("training supports act=relu or identity")
+        rows = max(s.out_row0 + s.n for s in segments)
+        H = agg.hidden_dim
+        with torch.no_grad():
+            used = agg._used_table(src, False)
+            Wh = kernel[agg.neigh_input_dim:]
+            neigh_h = torch.empty((rows, H), dtype=torch.float32, device=src.device)
+            kept = []
+            for s in segments:
+                X = agg.neighbour_rows(src, s)
+                P = agg._project(X)
+                _, kh, kc, lens = ops.lstm_seq(P, Wh, used, s.n, s.k,
+                                               row_ids=None if s.neigh_ids is None else s.neigh_ids[:s.n * s.k],
+                                               row0=s.neigh_row0, out=neigh_h[s.out_row0:s.out_row0 + s.n], keep=True)
+                kept.extend([X, P, kh, kc, lens])
+            xs = agg.self_rows(src, segments, rows)
+            y = agg._finish([(xs, agg.input_dim, Ws), (neigh_h, H, Wn)], agg._combine())
+        ctx.relu, ctx.concat, ctx.F_in = code == ops.ACT_RELU, bool(agg.concat), agg.neigh_input_dim
+        ctx.segments, ctx.src_shape = segments, tuple(src.shape)
+        ctx.src_needs_grad = bool(torch.is_tensor(src) and src.requires_grad)
+        ctx.save_for_backward(xs, neigh_h, y, Ws, Wn, kernel, *kept)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        xs, neigh_h, y, Ws, Wn, kernel = ctx.saved_tensors[:6]
+        kept = ctx.saved_tensors[6:]
+        dz = dy * (y > 0).to(dy.dtype) if ctx.relu else dy
+        D = Ws.shape[1]
+        dz_s, dz_n = (dz[:, :D], dz[:, D:]) if ctx.concat else (dz, dz)
+        dWs, dWn = xs.t() @ dz_s, neigh_h.t() @ dz_n
+        dneigh = dz_n @ Wn.t()
+        Wx, Wh = kernel[:ctx.F_in], kernel[ctx.F_in:]
+        dWx, dWh = torch.zeros_like(Wx), torch.zeros_like(Wh)
+        db = torch.zeros(kernel.shape[1], dtype=dy.dtype, device=dy.device)
+        dsrc = torch.zeros(ctx.src_shape, dtype=dy.dtype, device=dy.device) if ctx.src_needs_grad else None
+        dxs = dz_s @ Ws.t() if ctx.src_needs_grad else None
+        for i, s in enumerate(ctx.segments):
+            X, P, kh, kc, lens = kept[5 * i:5 * i + 5]
+            rows = slice(s.out_row0, s.out_row0 + s.n)
+            g_wx, g_wh, g_b, dX = lstm_seq_backward(P, X, Wx, Wh, kh, kc, lens, dneigh[rows], ctx.src_needs_grad)
+            dWx += g_wx
+            dWh += g_wh
+            db += g_b
+            if ctx.src_needs_grad:
+                if s.self_ids is not None or s.neigh_ids is not None:
+                    raise NotImplementedError("gradient w.r.t. an id-addressed source (trainable features) is out of scope")
+                dsrc[s.neigh_row0:s.neigh_row0 + s.n * s.k] += dX
+                dsrc[s.self_row0:s.self_row0 + s.n] += dxs[rows]
+        return None, dsrc, None, dWs, dWn, torch.cat([dWx, dWh], dim=0), db
+
+
 def differentiable_outputs(model, batch, normalize=True):
     """sample -> aggregate (-> l2_normalize) with an autograd graph over the aggregator weights; `model` is a
     SampleAndAggregate whose .aggregators exist (reference models.py:347-350 / supervised_models.py:79-85)."""
@@ -192,7 +291,10 @@ def differentiable_outputs(model, batch, normalize=True):
                 segs.append(ops.Seg(counts[hop], k, self_row0=row0[hop], neigh_row0=row0[hop + 1],
                                     out_row0=row0[hop]))
         agg = model.aggregators[layer]
-        if hasattr(agg, "mlp_layers"):                      # max-pool / mean-pool
+        if isinstance(agg, SeqAggregator):                  # LSTM
+            src = _SeqAggregateRowsFn.apply(agg, src, segs, agg.vars["self_weights"], agg.vars["neigh_weights"],
+                                            agg.cell_vars["kernel"], agg.cell_vars["bias"])
+        elif hasattr(agg, "mlp_layers"):                      # max-pool / mean-pool
             mlp = agg.mlp_layers[0].vars
             src = _PoolAggregateRowsFn.apply(agg, src, segs, agg.vars["self_weights"], agg.vars["neigh_weights"],
                                              mlp["weights"], mlp["bias"])
@@ -217,7 +319,8 @@ def build_aggregators(model):
     for layer in range(L):
         dim_mult = 2 if model.concat and layer != 0 else 1
         act = identity if layer == L - 1 else relu
-        extra = {"model_size": model.model_size} if hasattr(model.aggregator_cls, "pool") else {}
+        extra = {"model_size": model.model_size} if issubclass(model.aggregator_cls, (MaxPoolingAggregator, SeqAggregator)) \
+            else {}
         aggs.append(model.aggregator_cls(dim_mult * model.dims[layer], model.dims[layer + 1], act=act, dropout=0.,
                                          concat=model.concat, device=model.device, **extra))
     return aggs
@@ -226,9 +329,11 @@ def build_aggregators(model):
 def aggregator_parameters(aggregators):
     """(all trainable tensors, the subset the reference applies weight decay to).  The reference decays
     `aggregator.vars` only (supervised_models.py:103-105, models.py:385-387) - the pooling aggregators' Dense variables
-    live in `mlp_layers[0].vars` and are trained but not decayed."""
+    live in `mlp_layers[0].vars`, the seq aggregator's LSTM variables in `cell_vars` (the reference keeps them in the
+    cell); both are trained but not decayed."""
     decayed = [v for a in aggregators for v in a.vars.values()]
     extra = [v for a in aggregators for layer in getattr(a, "mlp_layers", []) for v in layer.vars.values()]
+    extra += [v for a in aggregators for v in getattr(a, "cell_vars", {}).values()]
     return decayed + extra, decayed
 
 
@@ -260,8 +365,8 @@ class SupervisedGraphsage(SampleAndAggregate):
         super(SupervisedGraphsage, self).__init__(placeholders, features, adj, degrees, layer_infos, concat=concat,
                                                   aggregator_type=aggregator_type, model_size=model_size,
                                                   identity_dim=identity_dim, device=device, **kwargs)
-        if aggregator_type not in ("mean", "gcn", "maxpool", "meanpool"):
-            raise NotImplementedError("training is implemented for the mean, gcn, maxpool and meanpool aggregators")
+        if aggregator_type not in ("mean", "gcn", "maxpool", "meanpool", "seq"):
+            raise NotImplementedError("training is implemented for the mean, gcn, maxpool, meanpool and seq aggregators")
         self.num_classes = num_classes
         self.sigmoid_loss = sigmoid_loss
         self.learning_rate, self.weight_decay = learning_rate, weight_decay

@@ -39,8 +39,8 @@ class UnsupervisedGraphsage(SampleAndAggregate):
         super(UnsupervisedGraphsage, self).__init__(placeholders, features, adj, degrees, layer_infos, concat=concat,
                                                     aggregator_type=aggregator_type, model_size=model_size,
                                                     identity_dim=identity_dim, device=device, **kwargs)
-        if aggregator_type not in ("mean", "gcn", "maxpool", "meanpool"):
-            raise NotImplementedError("training is implemented for the mean, gcn, maxpool and meanpool aggregators")
+        if aggregator_type not in ("mean", "gcn", "maxpool", "meanpool", "seq"):
+            raise NotImplementedError("training is implemented for the mean, gcn, maxpool, meanpool and seq aggregators")
         self.neg_sample_size, self.neg_sample_weights = int(neg_sample_size), float(neg_sample_weights)
         self.learning_rate, self.weight_decay = learning_rate, weight_decay
         self.neg_sampler = UnigramNegativeSampler(degrees, 0.75, seed, device)      # models.py:336-343

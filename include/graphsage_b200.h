@@ -355,6 +355,27 @@ int32_t gs_meanpool_mlp_fused(const void* table_bf16, int64_t n_rows, int32_t K,
                               float* out, int64_t ldo, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * SeqAggregator - the LSTM neighbour aggregator (reference graphsage/aggregators.py:363-449).
+ *   gs_row_used : used[r] = 1 if any of x[r, 0:F] is non-zero, else 0 - tf.sign(tf.reduce_max(tf.abs(x), axis=-1))
+ *       (aggregators.py:411).  dtype GS_F32 or GS_BF16; rows at stride `pitch`.
+ *   gs_lstm_seq : tf.nn.dynamic_rnn(BasicLSTMCell(H), neigh_vecs, sequence_length = len) followed by the gather of each
+ *       sequence's last valid output (aggregators.py:408-433), for n sequences of k steps in ONE launch:
+ *         len_g = max(1, sum_{t<k} used[row(g, t)]),  row(g, t) = row_ids ? row_ids[g*k + t] : row0 + g*k + t
+ *           (the count of non-zero rows; the recurrence still consumes the FIRST len_g rows, as dynamic_rnn does);
+ *         gates_t = P[g*k + t, 0:4H] + h_{t-1} @ Wh   (h_{-1} = c_{-1} = 0), column blocks i, j, f, o;
+ *         c_t = c_{t-1} * sigmoid(f + 1) + sigmoid(i) * tanh(j);  h_t = tanh(c_t) * sigmoid(o)   (forget_bias 1.0);
+ *         out[g, 0:H] = h_{len_g - 1}.
+ *       P is the input projection x_{g,t} @ kernel[0:in] + bias (fp32, row stride ldp >= 4H); Wh = kernel[in:in+H] is
+ *       fp32 [H, 4H] row-major.  keep_h / keep_c (fp32 [n, k, H], may be NULL) receive h_t / c_t for t < len_g (rows
+ *       t >= len_g are not written); lengths (int32 [n], may be NULL) receives len_g - the backward pass's inputs.
+ *       Exact fp32 arithmetic (FFMA, expf / tanhf).  GS_ERR_UNSUPPORTED unless H % 32 == 0 and H <= 256.
+ * --------------------------------------------------------------------------------------------- */
+int32_t gs_row_used(const void* x, int32_t dtype, int64_t n_rows, int32_t F, int64_t pitch, uint8_t* used, void* stream);
+int32_t gs_lstm_seq(const float* P, int64_t ldp, const float* Wh, int32_t H, const uint8_t* used, const int32_t* row_ids,
+                    int64_t row0, int64_t n, int32_t k, float* out, int64_t ldo, float* keep_h, float* keep_c,
+                    int32_t* lengths, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * One pipelined step from HOST buffers in a single call (no per-kernel host work), on three streams:
  *   h2d_stream     : wait ev_done (this slot's previous step no longer reads ids_dev), copy ids host->device,
  *                    record ev_ids
